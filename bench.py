@@ -56,6 +56,45 @@ def algorithmic_bytes(P, V, R, W, H):
     }
 
 
+DUMP_MAX_BYTES = 64 << 20
+DUMP_PIXELS = 1 << 18          # image planes larger than this are written at this many pixels, ...
+DUMP_SPLATS = 1 << 16          # ... per-splat arrays at this many splats
+
+
+def _dump_sample(n, k, seed):
+    """Sorted indices of a fixed, seeded sample of k out of n, or None when everything fits."""
+    import numpy as np
+    if n <= k:
+        return None
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+
+
+def dump_outputs(out_dir, images, per_splat):
+    """Writes one step's results as <out_dir>/<name>.npy (float32; sample indices float64).  images: name -> (C, H, W),
+    per_splat: name -> (P, ...).  At large sizes the images are reduced to (C, DUMP_PIXELS) columns of the flattened
+    H*W plane (pixel_index.npy) and the per-splat arrays to DUMP_SPLATS rows (splat_index.npy): the same indices
+    whenever the shapes are the same, so that two builds can be compared output for output."""
+    import numpy as np
+    H, W = next(iter(images.values())).shape[1:]
+    P = next(iter(per_splat.values())).shape[0]
+    pix, spl = _dump_sample(H * W, DUMP_PIXELS, 1), _dump_sample(P, DUMP_SPLATS, 2)
+    arrays = {}
+    for k, v in images.items():
+        arrays[k] = np.asarray(v, np.float32) if pix is None else np.asarray(v, np.float32).reshape(v.shape[0], -1)[:, pix]
+    for k, v in per_splat.items():
+        arrays[k] = np.asarray(v, np.float32) if spl is None else np.asarray(v, np.float32)[spl]
+    if pix is not None:
+        arrays["pixel_index"] = pix.astype(np.float64)
+    if spl is not None:
+        arrays["splat_index"] = spl.astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"{total} bytes of outputs to dump"
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), np.ascontiguousarray(a))
+    return sorted(arrays)
+
+
 def measured_peak():
     path = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(path):
@@ -537,12 +576,21 @@ def run_ours(args, rank, local_rank, world):
     host_ts = [time.perf_counter()]          # diagnostic only: when the host finished issuing each step
     e0.record()
     for _ in range(args.steps):
-        step(leaf, means2D, gc, go)
+        last = None           # free the previous step's outputs first: the allocator reuses their blocks, as without --dump-outputs
+        last = step(leaf, means2D, gc, go)
         host_ts.append(time.perf_counter())
     e1.record()
     torch.cuda.synchronize()
     sampler.mark_stop()
     _gc.enable()
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before the passes below overwrite the gradients
+        out_color, out_radii, out_allmap = last
+        grads = {f"grad_{k}": leaf[k].grad for k in names}
+        grads["grad_means2D"] = means2D.grad
+        dump_outputs(args.dump_outputs, {"color": out_color.detach().cpu().numpy(), "allmap": out_allmap.detach().cpu().numpy()},
+                     {"radii": out_radii.cpu().numpy(), **{k: g.cpu().numpy() for k, g in grads.items()}})
+    del last
     launches = int(lib.surfel_launch_count() - launches0)
     # second pass, same loop, with CUDA events recorded around every kernel on the launching stream:
     # per-kernel durations for the roofline (kept out of the pass that produces `value`)
@@ -754,7 +802,14 @@ def main():
     ap.add_argument("--pin-policy", choices=["local", "interleave"], default=os.environ.get("SURFEL_PIN_POLICY", "local"),
                     help="NUMA placement of the e2e leg's pinned host buffers")
     ap.add_argument("--no-tile-band", action="store_true", help="skip the tile-band leg that runs at N > 1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs and gradients (rank 0) as DIR/<name>.npy, at most 64 MB: "
+                         "a fixed, seeded sample of pixels and splats at large sizes")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs records the timed path of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,101 +1,107 @@
-"""Drop-in evidence that needs the reference checkout (build container only; skipped where
-/root/reference does not exist, e.g. on the GPU box): the reference's OWN GaussianModel code —
-training_setup, update_learning_rate, prune_points, densification_postfix, reset_opacity, capture/restore
-— is run with `diff_surfel_rasterization.optim.FusedAdam` substituted for torch.optim.Adam, and must leave
-the optimizer in exactly the state it leaves a torch.optim.Adam in.  (FusedAdam.step itself needs a GPU and is
-covered by tests/test_optim_gpu.py; here the per-parameter state is planted by hand, as Adam would create it.)
-Runs in a subprocess because the reference hard-codes device="cuda" and torch has to be patched to CPU."""
-import os
-import subprocess
-import sys
-import textwrap
+"""Drop-in evidence against the reference's own Python, through data it produced (tests/golden/ref_interop.npz,
+written by tests/golden/make_golden_interop.py from a checkout of the reference).
 
+  * The reference's densification code (training_setup, update_learning_rate, prune_points, densification_postfix,
+    reset_opacity, capture) manipulates its optimizer only through the torch.optim.Adam surface: it selects rows of
+    a group's parameter and of its Adam moments, appends rows with zero moments, and replaces a parameter with its
+    moments zeroed, each time re-keying optimizer.state to the new nn.Parameter.  The golden holds the optimizer as
+    that code left a torch.optim.Adam; the same operations applied to `diff_surfel_rasterization.optim.FusedAdam`
+    must leave it in exactly that state.  (FusedAdam.step itself needs a GPU and is covered by
+    tests/test_optim_gpu.py; here the per-parameter state is planted by hand, as Adam would create it.)
+  * The reference's unmodified gaussian_renderer.render() passes fixed keyword patterns to
+    GaussianRasterizationSettings(...) and GaussianRasterizer(...)(...) (compute_cov3D_python on/off x SH /
+    override_color inputs); the golden holds them verbatim and they must drive OUR Python surface down to the
+    native call, which is replaced here (no GPU)."""
+import json
+import os
+
+import numpy as np
 import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
-
-SCRIPT = textwrap.dedent('''
-    import sys, types
-    import torch
-    sys.path.insert(0, {root!r} + "/tests/golden"); sys.path.insert(0, {root!r}); sys.path.insert(0, {root!r} + "/2d-gaussian-splatting_b200")
-    from diff_surfel_rasterization.optim import FusedAdam           # the real package, before the stubs go in
-    import make_golden as MG
-    MG.cpu_patches(); MG.stub_modules({{}})                           # plyfile / simple_knn / ... stubs, torch -> CPU
-    sys.path.insert(0, {ref!r})
-    import scene.gaussian_model as GM
-
-    def build(adam_cls):
-        torch.optim.Adam, keep = adam_cls, torch.optim.Adam          # training_setup calls torch.optim.Adam(l, lr=0.0, eps=1e-15)
-        try:
-            g = torch.Generator("cpu").manual_seed(5)
-            P = 12
-            pc = GM.GaussianModel(3)
-            pc._xyz = torch.nn.Parameter(torch.randn(P, 3, generator=g))
-            pc._features_dc = torch.nn.Parameter(torch.randn(P, 1, 3, generator=g))
-            pc._features_rest = torch.nn.Parameter(torch.randn(P, 15, 3, generator=g))
-            pc._opacity = torch.nn.Parameter(torch.randn(P, 1, generator=g))
-            pc._scaling = torch.nn.Parameter(torch.randn(P, 2, generator=g))
-            pc._rotation = torch.nn.Parameter(torch.randn(P, 4, generator=g))
-            pc.max_radii2D = torch.zeros(P)
-            pc.spatial_lr_scale = 5.0
-            args = types.SimpleNamespace(percent_dense=0.01, position_lr_init=0.00016, position_lr_final=0.0000016,
-                                         position_lr_delay_mult=0.01, position_lr_max_steps=30000, feature_lr=0.0025,
-                                         opacity_lr=0.05, scaling_lr=0.005, rotation_lr=0.001)
-            pc.training_setup(args)
-        finally:
-            torch.optim.Adam = keep
-        opt = pc.optimizer
-        for grp in opt.param_groups:                                   # state as Adam creates it on the first step
-            p = grp["params"][0]
-            opt.state[p] = {{"step": torch.tensor(3.0), "exp_avg": torch.randn(p.shape, generator=g),
-                            "exp_avg_sq": torch.rand(p.shape, generator=g)}}
-        lr = pc.update_learning_rate(1000)
-        mask = torch.zeros(12, dtype=torch.bool); mask[[1, 4, 9]] = True
-        pc.prune_points(mask)
-        n = 4
-        pc.densification_postfix(torch.ones(n, 3), torch.ones(n, 1, 3), torch.ones(n, 15, 3), torch.ones(n, 1),
-                                 torch.ones(n, 2), torch.ones(n, 4))
-        pc.reset_opacity()
-        snap = pc.capture()                                            # checkpoint path: optimizer.state_dict()
-        return pc, lr, snap
-
-    a, lr_a, snap_a = build(torch.optim.Adam)
-    b, lr_b, snap_b = build(FusedAdam)
-    assert isinstance(b.optimizer, FusedAdam) and isinstance(b.optimizer, torch.optim.Adam)
-    assert lr_a == lr_b
-    for ga, gb in zip(a.optimizer.param_groups, b.optimizer.param_groups):
-        assert ga["name"] == gb["name"] and ga["lr"] == gb["lr"] and ga["eps"] == gb["eps"] == 1e-15 and ga["betas"] == gb["betas"]
-        pa, pb = ga["params"][0], gb["params"][0]
-        assert pa.shape == pb.shape and pa.shape[0] == 12 - 3 + 4 and torch.equal(pa, pb)
-        sa, sb = a.optimizer.state[pa], b.optimizer.state[pb]
-        assert set(sa) == set(sb) == {{"step", "exp_avg", "exp_avg_sq"}}
-        for k in sa:
-            assert torch.equal(sa[k], sb[k]), (ga["name"], k)
-    sd_a, sd_b = snap_a[-2], snap_b[-2]                                # optimizer.state_dict() inside capture()
-    assert sd_a["param_groups"][0].keys() == sd_b["param_groups"][0].keys() or set(sd_a["param_groups"][0]) <= set(sd_b["param_groups"][0])
-    b.optimizer.load_state_dict(sd_a)                                  # a checkpoint written with torch's Adam loads
-    print("INTEROP_OK", len(a.optimizer.param_groups))
-''')
+GOLD = os.path.join(ROOT, "tests", "golden", "ref_interop.npz")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (build container only)")
-def test_reference_densification_code_runs_unchanged_on_fused_adam():
-    r = subprocess.run([sys.executable, "-c", SCRIPT.format(root=ROOT, ref=REF)], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-3000:]
-    assert "INTEROP_OK 6" in r.stdout
+@pytest.fixture(scope="module")
+def gold():
+    return np.load(GOLD)
 
 
-RENDER_SCRIPT = textwrap.dedent('''
-    import sys, types
-    import numpy as np
-    import torch
-    sys.path.insert(0, {root!r} + "/tests/golden"); sys.path.insert(0, {root!r}); sys.path.insert(0, {root!r} + "/2d-gaussian-splatting_b200")
-    import diff_surfel_rasterization as real                       # OUR package: same import name as upstream's
-    import surfel_scenes as S
-    import make_golden as MG
-    MG.cpu_patches(); MG.stub_modules({{}})
-    sys.modules["diff_surfel_rasterization"] = real                # undo the rasterizer stub: the reference must import ours
+def _optimizer_as_the_reference_leaves_it(adam_cls, gold):
+    names = [str(n) for n in gold["opt_names"]]
+    lr0, eps = (float(x) for x in gold["opt_defaults"])
+    params = [torch.nn.Parameter(torch.from_numpy(gold[f"opt_init_{n}_param"].copy())) for n in names]
+    opt = adam_cls([{"params": [p], "lr": float(lr), "name": n} for p, lr, n in zip(params, gold["opt_init_lr"], names)],
+                   lr=lr0, eps=eps)
+    for grp in opt.param_groups:                                       # state as Adam creates it on the first step
+        n = grp["name"]
+        opt.state[grp["params"][0]] = {"step": torch.tensor(3.0),
+                                       "exp_avg": torch.from_numpy(gold[f"opt_init_{n}_exp_avg"].copy()),
+                                       "exp_avg_sq": torch.from_numpy(gold[f"opt_init_{n}_exp_avg_sq"].copy())}
+
+    def swap(grp, param_fn, moment_fn):
+        old = grp["params"][0]
+        st = opt.state.pop(old)
+        for k in ("exp_avg", "exp_avg_sq"):
+            st[k] = moment_fn(st[k])
+        grp["params"][0] = torch.nn.Parameter(param_fn(old.detach()).requires_grad_(True))
+        opt.state[grp["params"][0]] = st
+
+    for grp in opt.param_groups:                                       # update_learning_rate: the xyz group only
+        if grp["name"] == "xyz":
+            grp["lr"] = float(gold["opt_xyz_lr"])
+    keep = torch.from_numpy(~gold["opt_prune_mask"])
+    for grp in opt.param_groups:                                       # prune_points
+        swap(grp, lambda t: t[keep], lambda m: m[keep])
+    for grp in opt.param_groups:                                       # densification_postfix
+        ext = torch.from_numpy(gold[f"opt_append_{grp['name']}"].copy())
+        swap(grp, lambda t: torch.cat((t, ext)), lambda m: torch.cat((m, torch.zeros_like(ext))))
+    for grp in opt.param_groups:                                       # reset_opacity
+        if grp["name"] == "opacity":
+            new = torch.from_numpy(gold["opt_final_opacity_param"].copy())
+            swap(grp, lambda t: new, torch.zeros_like)
+    return opt
+
+
+def test_reference_densification_code_runs_unchanged_on_fused_adam(gold):
+    from diff_surfel_rasterization.optim import FusedAdam
+    arms = {cls.__name__: _optimizer_as_the_reference_leaves_it(cls, gold) for cls in (torch.optim.Adam, FusedAdam)}
+    assert isinstance(arms["FusedAdam"], torch.optim.Adam)
+    for arm, opt in arms.items():            # torch's own Adam as well: the replay itself must reproduce the reference
+        assert [g["name"] for g in opt.param_groups] == [str(n) for n in gold["opt_names"]], arm
+        for grp in opt.param_groups:
+            n, p = grp["name"], grp["params"][0]
+            assert grp["lr"] == float(gold[f"opt_final_{n}_lr"]) and grp["eps"] == float(gold[f"opt_final_{n}_eps"]) == 1e-15
+            assert tuple(grp["betas"]) == tuple(gold[f"opt_final_{n}_betas"]), (arm, n)
+            assert p.shape[0] == 12 - 3 + 4 and torch.equal(p.detach(), torch.from_numpy(gold[f"opt_final_{n}_param"])), (arm, n)
+            st = opt.state[p]
+            assert set(st) == {"step", "exp_avg", "exp_avg_sq"}, (arm, n)
+            for k in st:
+                assert torch.equal(st[k], torch.from_numpy(np.asarray(gold[f"opt_final_{n}_{k}"]))), (arm, n, k)
+    sd_ref = arms["Adam"].state_dict()
+    sd_fused = arms["FusedAdam"].state_dict()                          # capture(): optimizer.state_dict()
+    assert {str(k) for k in gold["opt_state_dict_group_keys"]} <= set(sd_fused["param_groups"][0])
+    assert set(sd_ref["param_groups"][0]) <= set(sd_fused["param_groups"][0])
+    arms["FusedAdam"].load_state_dict(sd_ref)                          # a checkpoint written with torch's Adam loads
+
+
+def _replayed(gold, i, part, meta):
+    kw = {}
+    for k, m in meta.items():
+        if m["kind"] == "tensor":
+            t = torch.from_numpy(np.asarray(gold[f"render{i}_{part}_{k}"]).copy())
+            assert str(t.dtype).replace("torch.", "") == m["dtype"], k
+            kw[k] = t.requires_grad_(m["requires_grad"])
+        else:
+            kw[k] = m["value"]
+    return kw
+
+
+def test_reference_render_drives_our_python_surface(gold, monkeypatch):
+    """Our GaussianRasterizationSettings and GaussianRasterizer accept the reference render()'s own keywords and
+    argument patterns; only the native call below the Python surface is replaced."""
+    import diff_surfel_rasterization as real
     calls = []
 
     def fake_native(means3D, means2D, sh, colors_precomp, opacities, scales, rotations, cov3Ds_precomp, rs):
@@ -103,53 +109,26 @@ RENDER_SCRIPT = textwrap.dedent('''
                           scales=scales, rotations=rotations, cov3Ds_precomp=cov3Ds_precomp, rs=rs))
         H, W = rs.image_height, rs.image_width
         return torch.zeros(3, H, W), torch.ones(means3D.shape[0], dtype=torch.int32), torch.ones(7, H, W)
-    real.rasterize_gaussians = fake_native                         # everything ABOVE the native call is the real code
-    sys.path.insert(0, {ref!r})
-    from gaussian_renderer import render                           # /root/reference/gaussian_renderer/__init__.py:14 imports ours
-    from scene.cameras import Camera
-    from scene.gaussian_model import GaussianModel
-
-    W, H, P = 64, 48, 10
-    Rm, tv = S.look_at_rotation(10, 5), np.array([0.1, 0.0, 0.3])
-    mycam = S.make_camera(W, H, R=Rm, t=tv)
-    cam = Camera(colmap_id=0, R=Rm, T=tv, FoVx=mycam["FoVx"], FoVy=mycam["FoVy"], image=torch.zeros(3, H, W),
-                 gt_alpha_mask=None, image_name="g", uid=0, data_device="cpu")
-    scene = S.make_scene(P, W, H, 4, depth_complexity=2)
-    pc = GaussianModel(3); pc.active_sh_degree = 3
-    pc._xyz, pc._scaling, pc._rotation = scene["means3D"], torch.log(scene["scales"]), scene["rotations"]
-    pc._opacity = torch.log(scene["opacities"] / (1 - scene["opacities"]))
-    pc._features_dc, pc._features_rest = scene["shs"][:, :1].contiguous(), scene["shs"][:, 1:].contiguous()
-    for cov_py in (False, True):
-        for sh_py in (False, True):
-            # render() forces pipe.convert_SHs_python = False (gaussian_renderer/__init__.py:82): its colors_precomp
-            # path is reached through override_color
-            pipe = types.SimpleNamespace(compute_cov3D_python=cov_py, convert_SHs_python=False, depth_ratio=0.0, debug=False)
-            rets = render(cam, pc, pipe, torch.zeros(3), override_color=torch.rand(P, 3) if sh_py else None)
-            c = calls[-1]
-            rs = c["rs"]
-            assert isinstance(rs, real.GaussianRasterizationSettings)
-            assert (rs.image_height, rs.image_width, rs.sh_degree, rs.prefiltered, rs.scale_modifier) == (H, W, 3, False, 1.0)
-            assert isinstance(rs.tanfovx, float) and rs.viewmatrix.shape == (4, 4) and rs.projmatrix.shape == (4, 4) and rs.campos.shape == (3,)
-            assert c["means3D"].shape == (P, 3) and c["means2D"].shape == (P, 3) and c["opacities"].shape == (P, 1)
-            assert (c["cov3Ds_precomp"].numel() > 0) == cov_py and (c["scales"].numel() > 0) == (not cov_py) and (c["rotations"].numel() > 0) == (not cov_py)
-            assert (c["colors_precomp"].numel() > 0) == sh_py and (c["sh"].numel() > 0) == (not sh_py)
-            if cov_py:
-                assert c["cov3Ds_precomp"].shape == (P, 9)
-            if not sh_py:
-                assert c["sh"].shape == (P, 16, 3)
-            assert set(rets) >= {{"render", "viewspace_points", "visibility_filter", "radii", "rend_alpha", "rend_normal",
-                                 "rend_dist", "surf_depth", "surf_normal"}}
-            assert rets["visibility_filter"].dtype == torch.bool and rets["visibility_filter"].all()
-    print("RENDER_INTEROP_OK", len(calls))
-''')
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (build container only)")
-def test_reference_render_drives_our_python_surface():
-    """The reference's unmodified gaussian_renderer.render() imports OUR diff_surfel_rasterization, builds
-    GaussianRasterizationSettings with its own keywords and calls GaussianRasterizer with its own argument patterns
-    (compute_cov3D_python on/off x SH / override_color inputs); only the native call below the Python surface
-    is replaced (no GPU here)."""
-    r = subprocess.run([sys.executable, "-c", RENDER_SCRIPT.format(root=ROOT, ref=REF)], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-3000:]
-    assert "RENDER_INTEROP_OK 4" in r.stdout
+    monkeypatch.setattr(real, "rasterize_gaussians", fake_native)
+    meta = json.loads(str(gold["render_meta"]))
+    assert [(m["cov3D_python"], m["override_color"]) for m in meta] == [(False, False), (False, True), (True, False), (True, True)]
+    for i, m in enumerate(meta):
+        cov_py, sh_py = m["cov3D_python"], m["override_color"]
+        rs_in = real.GaussianRasterizationSettings(**_replayed(gold, i, "settings", m["settings"]))
+        color, radii, allmap = real.GaussianRasterizer(raster_settings=rs_in)(**_replayed(gold, i, "call", m["call"]))
+        c = calls[-1]
+        rs = c["rs"]
+        P = c["means3D"].shape[0]
+        H, W = rs.image_height, rs.image_width
+        assert isinstance(rs, real.GaussianRasterizationSettings)
+        assert (H, W, rs.sh_degree, rs.prefiltered, rs.scale_modifier) == (48, 64, 3, False, 1.0)
+        assert isinstance(rs.tanfovx, float) and rs.viewmatrix.shape == (4, 4) and rs.projmatrix.shape == (4, 4) and rs.campos.shape == (3,)
+        assert P == 10 and c["means2D"].shape == (P, 3) and c["opacities"].shape == (P, 1)
+        assert (c["cov3Ds_precomp"].numel() > 0) == cov_py and (c["scales"].numel() > 0) == (not cov_py) and (c["rotations"].numel() > 0) == (not cov_py)
+        assert (c["colors_precomp"].numel() > 0) == sh_py and (c["sh"].numel() > 0) == (not sh_py)
+        if cov_py:
+            assert c["cov3Ds_precomp"].shape == (P, 9)
+        if not sh_py:
+            assert c["sh"].shape == (P, 16, 3)
+        assert color.shape == (3, H, W) and allmap.shape == (7, H, W) and radii.shape == (P,) and radii.dtype == torch.int32
+    assert len(calls) == 4
